@@ -2,6 +2,7 @@
 """Benchmark of the dqn_zoo hot path (replay sample -> learner update -> priority write-back).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--agent rainbow|dqn|c51|iqn|...]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
       bench.py --gpus N --steps K --warmup W
 
@@ -13,6 +14,8 @@ transitions/s = x batch) on a synthetic 84x84x4 uint8 replay of 1M transitions, 
 `roofline`: the dominant kernel of the step, timed with CUDA events on its stream (dz_profile_*).
 `cpu_baseline` / `--impl reference`: the oracle PORT of the reference algorithm on the host cores
 (JAX is not installable here or on the GPU box; see oracle/cpu_reference.py).
+`--dump-outputs DIR`: after the timed steps, the results of the last timed step as DIR/<name>.npy (see dump_outputs), so
+that two builds run with the same arguments, hence the same inputs, can be compared output for output.
 """
 
 import argparse
@@ -53,7 +56,11 @@ def parse():
   ap.add_argument('--no-graph', action='store_true')
   ap.add_argument('--no-cpu-baseline', action='store_true')
   ap.add_argument('--cpu-steps', type=int, default=40)
-  return ap.parse_args()
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None)
+  args = ap.parse_args()
+  if args.dump_outputs and args.impl != 'ours':
+    ap.error('--dump-outputs writes the results of the CUDA path (--impl ours)')
+  return args
 
 
 def workload_name(args):
@@ -139,7 +146,7 @@ def reference_arm(args, rank, world):
   from oracle import cpu_reference
   steps, warmup = max(1, args.steps), max(0, args.warmup)
   res = cpu_reference.run(args.agent, capacity=args.capacity, batch=args.batch, steps=steps, warmup=warmup, seed=args.seed,
-                          threads='auto', prewarm=10, budget_s=100.0)
+                          threads='auto', prewarm=10, budget_s=None)
   value = res['steps_per_s']
   sample = ('%d learner steps (replay.sample + update + update_priorities) of %s after %d warm-up (+10 pre-warm) steps; replay '
             '%.2f ms + learner %.2f ms per step; observations reference a pool of 512 synthetic frames'
@@ -195,6 +202,30 @@ def build_agent(args, rank, device):
   else:
     ag = agent_lib.AGENTS[kind](exploration_epsilon=eps, grad_error_bound=1.0 / 32, **common)
   return ag, rep
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, ag, L, prioritized):
+  """Writes what the last learner step returned to its caller, as float32 / float64 .npy files: the loss, the per-example
+  loss, the new priorities, the global gradient norm, the sampled ids (as float64, exact below 2^53) and importance
+  weights, the updated online parameters and, with prioritized replay, the sum-tree leaves of the sampled transitions after
+  the priority write-back, the tree's root and the running max priority."""
+  arrays = {'loss': L.loss, 'per_example_loss': L.per_example, 'priorities': L.priorities, 'grad_norm': L.grad_norm,
+            'sampled_ids': L.sampled_ids.double(), 'importance_weights': L.sampled_weights, 'online_params': L.online}
+  if prioritized:
+    tree = ag._replay._distribution._sum_tree
+    arrays['sum_tree_leaves_sampled'] = tree._nodes[tree._first_leaf + L.sampled_indices]
+    arrays['sum_tree_root'] = tree._nodes[1:2]
+    arrays['max_seen_priority'] = L.max_seen_priority
+  arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+  total = sum(a.nbytes for a in arrays.values())
+  assert total <= DUMP_LIMIT_BYTES, 'outputs of %d bytes exceed the dump limit' % total
+  os.makedirs(out_dir, exist_ok=True)
+  for name, a in arrays.items():
+    assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+    np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 _REAL_STDOUT = None
@@ -282,6 +313,9 @@ def main():
   barrier()
   clk = clocks.stop()
   ms = e0.elapsed_time(e1)
+  if args.dump_outputs and rank == 0:
+    ag.check_device_flags()   # a step that set an error flag leaves no outputs behind that look valid
+    dump_outputs(args.dump_outputs, ag, L, AGENT_SETUP[args.agent][0])
   collective_us = 1e3 * float(np.mean([a.elapsed_time(b) for a, b in coll_events])) if coll_events else None
   t = torch.tensor([ms], dtype=torch.float64, device=device)
   if dist is not None:

@@ -116,7 +116,8 @@ def pick_threads(learner, make_inputs, limit):
 
 def run(kind='rainbow', capacity=1000000, batch=32, steps=20, warmup=3, seed=1, threads=None, budget_s=60.0, prewarm=0):
   """Returns dict(steps_per_s, replay_ms, learner_ms, steps, cores).  threads: an int, None (torch default) or 'auto'
-  (calibrated thread count within the CPUs this process may use)."""
+  (calibrated thread count within the CPUs this process may use).  budget_s: wall-clock seconds after which the timed
+  steps stop early; None runs all `steps`."""
   t_start = time.perf_counter()
   if threads and threads != 'auto':
     torch.set_num_threads(threads)
@@ -181,9 +182,9 @@ def run(kind='rainbow', capacity=1000000, batch=32, steps=20, warmup=3, seed=1, 
     t_learn += t2 - t1
     if it >= warmup:
       done += 1
-      if time.perf_counter() - t_begin > budget_s:
+      if budget_s is not None and time.perf_counter() - t_begin > budget_s:
         break
-    elif time.perf_counter() - t_start > 2.0 * budget_s and it + 1 < warmup:
+    elif budget_s is not None and time.perf_counter() - t_start > 2.0 * budget_s and it + 1 < warmup:
       warmup = it + 1          # a pathologically slow host: stop warming up, time what the budget allows
   wall = time.perf_counter() - t_begin
   return {'steps_per_s': done / wall, 'replay_ms': 1e3 * t_replay / done, 'learner_ms': 1e3 * t_learn / done,

@@ -1,7 +1,11 @@
-"""Generates tests/golden/replay_*.npz by running oracle/scenarios.py against the
-REFERENCE's own replay.py (imported from /root/reference, build container only).
+"""Generates the replay fixtures under tests/golden/ by running the REFERENCE's own
+replay.py (imported by oracle/ref_import.py from a checkout of the original dqn_zoo):
 
-  python -m oracle.gen_golden
+  replay_*.npz                    oracle/scenarios.py's scripts (ALL and LONG_PER_RUN)
+  replay_contract_reference.xz    every answer the reference gave to the checks of
+                                  tests/replay_contract.py (oracle/call_log.py)
+
+  DQN_ZOO_REFERENCE=<checkout of dqn_zoo> python -m oracle.gen_golden
 
 TEST INFRASTRUCTURE ONLY.  The fixtures are committed; this script is committed
 so they can be regenerated and audited.
@@ -22,8 +26,10 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
+sys.path.insert(0, os.path.join(os.path.dirname(HERE), 'tests'))
 
-from oracle import ref_import, replay_oracle, scenarios  # noqa: E402
+from oracle import call_log, ref_import, replay_oracle, scenarios  # noqa: E402
+import replay_contract  # noqa: E402
 
 
 def main():
@@ -31,12 +37,22 @@ def main():
   out_dir = os.path.join(os.path.dirname(HERE), 'tests', 'golden')
   os.makedirs(out_dir, exist_ok=True)
   stock_power = ref._power
-  for name, fn in scenarios.ALL.items():
+  runs = dict(scenarios.ALL)
+  runs['replay_per_long_random'] = lambda lib: scenarios.prioritized_replay_script(lib, **scenarios.LONG_PER_RUN)
+  for name, fn in runs.items():
     ref._power = replay_oracle.power_keep_zero if 'pow06' in name else stock_power
     res = fn(ref)
     np.savez_compressed(os.path.join(out_dir, name + '.npz'), **res)
     print(name, {k: tuple(v.shape) for k, v in res.items()})
   ref._power = stock_power
+  logs = {}
+  for check in replay_contract.CONTRACT:
+    rec = call_log.Recorder(ref)
+    check(rec)
+    logs[check.__name__] = rec.log
+  path = os.path.join(out_dir, 'replay_contract_reference.xz')
+  call_log.save(path, logs)
+  print('replay_contract_reference', {k: len(v) for k, v in logs.items()}, os.path.getsize(path), 'bytes')
 
 
 if __name__ == '__main__':

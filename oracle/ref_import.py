@@ -1,9 +1,8 @@
-"""Import the REFERENCE's own `dqn_zoo/replay.py` (build container only).
+"""Import the REFERENCE's own `dqn_zoo/replay.py` from a checkout of the original dqn_zoo (DQN_ZOO_REFERENCE).
 
-TEST INFRASTRUCTURE ONLY.  /root/reference does not exist on the GPU box, so
-nothing under tests/ -m gpu, smoke() or bench.py may call this; it is used by
-`oracle/gen_golden.py` (fixture generation) and by the CPU-only cross-check in
-`tests/test_oracle_replay.py`, which skips when the reference is absent.
+TEST INFRASTRUCTURE ONLY.  Used by `oracle/gen_golden.py` alone, to generate
+the fixtures under tests/golden/; the tests, smoke() and bench.py read those
+fixtures and never need the reference itself.
 
 `replay.py` only needs numpy + stdlib for its arithmetic; its three imports
 that are missing from this image are stubbed in `sys.modules`:
@@ -17,7 +16,7 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get('DQN_ZOO_REFERENCE', '/root/reference')
+REFERENCE_ROOT = os.environ.get('DQN_ZOO_REFERENCE', '')
 
 
 def available():
@@ -27,7 +26,7 @@ def available():
 def load_reference_replay():
   """Returns the reference `dqn_zoo.replay` module object, unmodified."""
   if not available():
-    raise RuntimeError('reference not mounted at %s' % REFERENCE_ROOT)
+    raise RuntimeError('no dqn_zoo/replay.py under DQN_ZOO_REFERENCE=%r' % REFERENCE_ROOT)
   saved = {k: sys.modules.get(k) for k in ('dm_env', 'snappy', 'dqn_zoo', 'dqn_zoo.parts')}
   try:
     dm_env = types.ModuleType('dm_env')

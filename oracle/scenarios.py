@@ -223,3 +223,6 @@ ALL = collections.OrderedDict([
     ('replay_nstep3', lambda lib: n_step_script(lib, n=3)),
     ('replay_nstep1', lambda lib: n_step_script(lib, n=1, seed=17)),
 ])
+
+# a longer PER run (wraps a 257-slot ring ~7 times), compared with the reference's result in replay_per_long_random.npz
+LONG_PER_RUN = dict(capacity=257, alpha=0.5, usp=1e-3, normalize=True, batch=32, rounds=400, seed=31)
