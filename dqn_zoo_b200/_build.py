@@ -8,7 +8,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB_DIR = os.path.join(HERE, 'lib')
 LIB_PATH = os.path.join(LIB_DIR, 'libdqnzoo_b200.so')
-SOURCES = ['dz_replay.cu', 'dz_learner.cu', 'dz_tcp.cu', 'dz_umma.cu', 'dz_umma_net.cu', 'dz_preprocess.cu', 'dz_jaxprng.cu']
+SOURCES = ['dz_replay.cu', 'dz_frames.cu', 'dz_learner.cu', 'dz_tcp.cu', 'dz_umma.cu', 'dz_umma_net.cu', 'dz_preprocess.cu', 'dz_jaxprng.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
               '-Xcompiler', '-fPIC', '--expt-relaxed-constexpr']
 

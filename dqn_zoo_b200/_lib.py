@@ -13,20 +13,29 @@ i32, i64, f32, f64, u64 = C.c_int32, C.c_int64, C.c_float, C.c_double, C.c_uint6
 vp = C.c_void_p
 
 DZ_FLAG_BAD_VALUE, DZ_FLAG_BAD_INDEX, DZ_FLAG_BAD_TARGET, DZ_FLAG_ROOT_ZERO, DZ_FLAG_NONFINITE_WEIGHT = 1, 2, 4, 8, 16
+DZ_FLAG_FRAME_POOL_FULL = 32
+DZ_FRAME_WINDOW, DZ_FRAME_MAX_STACK, DZ_FRAME_MAX_STAGE_BYTES = 16, 8, 200 * 1024
 AGENT_KINDS = {'dqn': 0, 'double_q': 1, 'prioritized': 2, 'c51': 3, 'qrdqn': 4, 'rainbow': 5, 'iqn': 6}
 OPTIMIZERS = {'adam': 0, 'rmsprop': 1}
+
+
+class FrameStore(C.Structure):
+  _fields_ = [('d_frames', vp), ('d_row_frames', vp), ('d_frame_hash', vp), ('d_frame_born', vp),
+              ('d_frame_last_ref', vp), ('d_state', vp), ('d_add_stage', vp), ('d_batch_stage', vp), ('num_frames', i64),
+              ('frame_bytes', i64), ('frame_stride', i64), ('stack', i32), ('batch_capacity', i32)]
 
 
 class ReplayView(C.Structure):
   _fields_ = [('d_obs', vp), ('d_action', vp), ('d_reward', vp), ('d_discount', vp), ('capacity', i64),
               ('obs_bytes', i64), ('obs_stride', i64), ('d_tree', vp), ('first_leaf', i64), ('d_live', vp),
-              ('d_id_at', vp), ('d_ids', vp), ('d_flags', vp)]
+              ('d_id_at', vp), ('d_ids', vp), ('d_flags', vp), ('frames', FrameStore)]
 
 
 class AddRecord(C.Structure):
   _fields_ = [('slot', i64), ('action', i32), ('reward', f64), ('discount', f64), ('n_patches', i32),
               ('patch_pos', i64 * 4), ('patch_val', i64 * 4), ('patch_target', i32 * 4), ('tree_index', i64),
-              ('leaf_value', f64), ('evict_index', i64), ('size_after', i64), ('d_priority', vp), ('alpha', f64)]
+              ('leaf_value', f64), ('evict_index', i64), ('size_after', i64), ('d_priority', vp), ('alpha', f64),
+              ('item_id', i64), ('oldest_live', i64)]
 
 
 class SampleInputs(C.Structure):
@@ -92,6 +101,8 @@ _SIGNATURES = {
     'dz_sumtree_get': (i32, [vp, i64, i64, vp, i64, vp, vp, vp]),
     'dz_replay_add': (i32, [C.POINTER(ReplayView), C.POINTER(AddRecord), vp, vp, vp]),
     'dz_replay_fill_synthetic': (i32, [C.POINTER(ReplayView), i64, i64, u64, i32, f64, vp]),
+    'dz_replay_fill_synthetic_frames': (i32, [C.POINTER(ReplayView), i64, i64, u64, i32, f64, vp]),
+    'dz_test_frame_hash': (i32, [vp, i64, vp]),
     'dz_replay_sample': (i32, [C.POINTER(ReplayView), i32, C.POINTER(SampleInputs), C.POINTER(SampleOutputs), i32, vp]),
     'dz_replay_gather': (i32, [C.POINTER(ReplayView), vp, i32, vp, vp, vp, vp, vp, vp]),
     'dz_replay_update_priorities': (i32, [C.POINTER(ReplayView), vp, vp, i32, f64, i64, vp]),

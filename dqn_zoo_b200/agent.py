@@ -60,6 +60,7 @@ class _DeviceAgent(parts.Agent):
                        % (np.asarray(sample_network_input).shape, network.obs_shape))
     self._preprocessor = preprocessor
     self._replay = replay
+    replay.reserve_batch(batch_size)          # before the first view: the staging address is part of a captured graph
     self._transition_accumulator = transition_accumulator
     self._batch_size = batch_size
     self._exploration_epsilon = exploration_epsilon
@@ -300,6 +301,9 @@ class _DeviceAgent(parts.Agent):
     f = int(flags.item())
     if f:
       flags.zero_()
+      if f & _lib.DZ_FLAG_FRAME_POOL_FULL:
+        raise RuntimeError('frame pool is full: frame_capacity is too small for the frames the live transitions '
+                           'reference (device flags %d).' % f)
       if f & (_lib.DZ_FLAG_BAD_VALUE | _lib.DZ_FLAG_BAD_INDEX):
         raise ValueError('value must be finite and positive, index in range (device flags %d).' % f)
       if f & _lib.DZ_FLAG_NONFINITE_WEIGHT:

@@ -21,6 +21,18 @@ int launch_sample(const dz_replay_view* view, int prioritized, const dz_sample_i
                   int batch, const BatchExtras& ex, void* stream);
 int launch_update_priorities(const dz_replay_view* view, const int64_t* d_indices, const float* d_priorities, int n,
                              double alpha, int64_t size, void* stream);
+int launch_fill_scalars(const dz_replay_view* view, int64_t row0, int64_t n, uint64_t seed, int num_actions,
+                        double discount, void* stream);
+
+// ---- frame-deduplicated storage (dz_frames.cu) ------------------------------------------------------------------
+bool frame_store_on(const dz_replay_view* v);
+// Every argument check of frames_insert; dz_replay_add runs it before it enqueues anything for the add.
+int frames_check_add(const dz_replay_view* v, const dz_add_record* rec);
+// The insert of one add whose two stacks are already in v->frames.d_add_stage.
+int frames_insert(const dz_replay_view* v, const dz_add_record* rec, void* stream);
+// HWC stacks of rows d_slots[0..batch): s_tm1 of row b at dst0 + b * pitch, s_t at dst1 + b * pitch.
+int launch_frame_assemble(const dz_replay_view* v, const int64_t* d_slots, int batch, uint8_t* dst0, uint8_t* dst1,
+                          int64_t pitch, void* stream);
 
 
 // ---- packed-operand tcgen05 GEMM (dz_tcp.cuh / dz_tcp.cu) ------------------------------------------------------

@@ -2674,6 +2674,9 @@ int dz_learner_learn(dz_learner* l, const dz_replay_view* replay, int32_t priori
   const int B = l->B;
   BatchExtras ex{l->rows_sample[0], l->rows_sample[1], l->s_a, l->s_r, l->s_d, prioritized ? l->s_w : nullptr, 1};
   if (replay->obs_bytes != (int64_t)l->d.H * l->d.W * l->d.C) return fail(DZ_EINVAL, "replay observation size does not match the network");
+  const bool frames = frame_store_on(replay);
+  if (frames && (B > replay->frames.batch_capacity || !replay->frames.d_batch_stage))
+    return fail(DZ_EINVAL, "batch exceeds the frame store's reserved batch staging");
   // conv weight images do not depend on the sampled batch: pack them on the side stream while the sampler runs
   const bool pack_aside = l->um != nullptr && l->side != nullptr;
   if (pack_aside) {
@@ -2681,6 +2684,11 @@ int dz_learner_learn(dz_learner* l, const dz_replay_view* replay, int32_t priori
     DZ_TRY(um_pack_weights(l->um, ws));
   }
   DZ_TRY(launch_sample(replay, prioritized, &io->sample_in, &io->sample_out, B, ex, stream));
+  if (frames) {   // the row tables point at the staging rows; fill them from the sampled rows' frame slots
+    uint8_t* stage = replay->frames.d_batch_stage;
+    DZ_TRY(launch_frame_assemble(replay, io->sample_out.d_slots, B, stage,
+                                 stage + (int64_t)replay->frames.batch_capacity * replay->obs_stride, replay->obs_stride, stream));
+  }
   dz_batch batch;
   batch.d_s_tm1_rows = l->rows_sample[0];
   batch.d_s_t_rows = l->rows_sample[1];

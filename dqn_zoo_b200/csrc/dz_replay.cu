@@ -293,9 +293,15 @@ __device__ __forceinline__ double is_weight_pow(double x, double beta) {
 }
 
 __device__ void emit_batch_rows(const dz_replay_view& v, const BatchExtras& ex, int b, int64_t slot, double weight) {
-  const uint8_t* row = v.d_obs + slot * 2 * v.obs_stride;
-  if (ex.d_s_tm1_rows) ex.d_s_tm1_rows[b] = row;
-  if (ex.d_s_t_rows) ex.d_s_t_rows[b] = row + v.obs_stride;
+  if (v.frames.d_frames) {   // frame store: the stacks are assembled into fixed staging rows after the sampler
+    const uint8_t* row = v.frames.d_batch_stage + (int64_t)b * v.obs_stride;
+    if (ex.d_s_tm1_rows) ex.d_s_tm1_rows[b] = row;
+    if (ex.d_s_t_rows) ex.d_s_t_rows[b] = row + (int64_t)v.frames.batch_capacity * v.obs_stride;
+  } else {
+    const uint8_t* row = v.d_obs + slot * 2 * v.obs_stride;
+    if (ex.d_s_tm1_rows) ex.d_s_tm1_rows[b] = row;
+    if (ex.d_s_t_rows) ex.d_s_t_rows[b] = row + v.obs_stride;
+  }
   if (ex.d_a) ex.d_a[b] = v.d_action[slot];
   if (ex.d_r) ex.d_r[b] = (float)v.d_reward[slot];      // float64 -> float32 at the jit boundary
   if (ex.d_disc) ex.d_disc[b] = (float)v.d_discount[slot];
@@ -516,6 +522,13 @@ int launch_sample(const dz_replay_view* view, int prioritized, const dz_sample_i
   return DZ_OK;
 }
 
+int launch_fill_scalars(const dz_replay_view* view, int64_t row0, int64_t n, uint64_t seed, int num_actions,
+                        double discount, void* stream) {
+  if (n <= 0) return DZ_OK;
+  DZ_LAUNCH(fill_scalars_kernel, (int)ceil_div(n, 256), 256, 0, stream, *view, row0, n, seed, num_actions, discount);
+  return DZ_OK;
+}
+
 int launch_update_priorities(const dz_replay_view* view, const int64_t* d_indices, const float* d_priorities, int n,
                              double alpha, int64_t size, void* stream) {
   if (n <= 32 && view->first_leaf >= 2) {
@@ -630,6 +643,16 @@ int dz_replay_add(const dz_replay_view* view, const dz_add_record* rec, const ui
                   void* stream) {
   if (rec->slot < 0 || rec->slot >= view->capacity) return fail(DZ_ERANGE, "slot out of range");
   if (rec->n_patches < 0 || rec->n_patches > 4) return fail(DZ_EINVAL, "at most 4 patches");
+  if (frame_store_on(view)) {   // both stacks go to the add staging area; frames_insert deduplicates their planes
+    if (!h_s_tm1 || !h_s_t) return fail(DZ_EINVAL, "a frame store add needs both observations");
+    int st = frames_check_add(view, rec);   // rejected before any copy or index patch is enqueued
+    if (st != DZ_OK) return st;
+    uint8_t* stage = view->frames.d_add_stage;
+    DZ_CUDA_OK(cudaMemcpyAsync(stage, h_s_tm1, view->obs_bytes, cudaMemcpyDefault, (cudaStream_t)stream));
+    DZ_CUDA_OK(cudaMemcpyAsync(stage + view->obs_stride, h_s_t, view->obs_bytes, cudaMemcpyDefault, (cudaStream_t)stream));
+    DZ_LAUNCH(apply_add_kernel, 1, 64, 0, stream, *view, *rec);
+    return frames_insert(view, rec, stream);
+  }
   uint8_t* row = view->d_obs + rec->slot * 2 * view->obs_stride;
   // cudaMemcpyDefault: the sources may be host arrays (the reference's add path) or device buffers (frame stacks kept
   // in HBM by the device preprocessing) — the driver infers the direction from the unified address space
@@ -661,6 +684,12 @@ int dz_replay_sample(const dz_replay_view* view, int32_t prioritized, const dz_s
 int dz_replay_gather(const dz_replay_view* view, const int64_t* d_slots, int32_t batch, uint8_t* d_s_tm1, uint8_t* d_s_t,
                      int64_t* d_a, double* d_r, double* d_disc, void* stream) {
   if (batch <= 0) return DZ_OK;
+  if (frame_store_on(view)) {
+    int st = launch_frame_assemble(view, d_slots, batch, d_s_tm1, d_s_t, view->obs_bytes, stream);
+    if (st != DZ_OK) return st;
+    DZ_LAUNCH(gather_scalars_kernel, (int)ceil_div(batch, 128), 128, 0, stream, *view, d_slots, batch, d_a, d_r, d_disc);
+    return DZ_OK;
+  }
   int vec16 = (view->obs_bytes % 16 == 0) && ((uintptr_t)d_s_tm1 % 16 == 0) && ((uintptr_t)d_s_t % 16 == 0);
   int64_t work = vec16 ? view->obs_bytes >> 4 : view->obs_bytes;
   int gx = (int)(ceil_div(work, 256) < 8 ? ceil_div(work, 256) : 8);

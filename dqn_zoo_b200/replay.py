@@ -8,7 +8,9 @@ generators.  What else differs is where things live:
 
   * transition storage (`OrderedDict` in the reference, `replay.py:140,688`) is a
     transition-major uint8 array in device memory: row = id % capacity holds
-    s_tm1 | s_t back to back (DESIGN.md §3);
+    s_tm1 | s_t back to back (DESIGN.md §3); with `frame_capacity=F` the row holds frame
+    slot numbers instead and every distinct (H, W) frame of the stacks is stored once
+    (`_FrameStore`), with byte-identical results;
   * the float64 sum tree (`replay.py:246-426`) is a device array traversed by a
     warp-cooperative CUDA kernel (csrc/dz_replay.cu);
   * O(1) integer bookkeeping per add (free-slot stack, swap-remove lists,
@@ -33,6 +35,8 @@ import torch
 
 from dqn_zoo_b200 import _lib
 
+_POOL_FULL_MESSAGE = ('frame pool is full: frame_capacity is too small for the frames the live transitions reference '
+                      '(the transitions added since are not stored)')
 _FLAG_NAMES = {1: 'value must be finite and positive', 2: 'index out of range', 4: 'Require 0 <= target < total sum.',
                8: 'sum-tree root is zero in the fused path', 16: 'Weights are not finite'}
 
@@ -107,6 +111,8 @@ class SumTree:
     f = int(self._flags.item())
     if f:
       self._flags.zero_()
+      if f & _lib.DZ_FLAG_FRAME_POOL_FULL:
+        raise RuntimeError(_POOL_FULL_MESSAGE)
       if f & _lib.DZ_FLAG_BAD_INDEX:
         raise IndexError('index out of range, expect 0 <= index < %s' % self._size)
       raise ValueError(_FLAG_NAMES.get(f & -f, 'device flag %d' % f))
@@ -271,9 +277,11 @@ class _DeviceList:
 
 
 def _apply_index_record(view, patches, tree_index=-1, leaf_value=0.0, evict_index=-1, size_after=0, slot=0,
-                        action=0, reward=0.0, discount=0.0, h_s_tm1=None, h_s_t=None, d_priority=None, alpha=1.0):
+                        action=0, reward=0.0, discount=0.0, h_s_tm1=None, h_s_t=None, d_priority=None, alpha=1.0,
+                        item_id=0, oldest_live=0):
   """One dz_replay_add call: <=4 list patches + optional evict/set on the tree (+ optional row write)."""
   rec = _lib.AddRecord()
+  rec.item_id, rec.oldest_live = item_id, oldest_live
   rec.slot, rec.action, rec.reward, rec.discount = slot, action, reward, discount
   rec.n_patches = len(patches)
   for k, (target, pos, val) in enumerate(patches):
@@ -707,6 +715,20 @@ class _TransitionStore:
     v.d_flags = _ptr(self.flags)
     return v
 
+  def reserve_batch(self, batch_size):
+    """Staging for the fused learner's batch (the frame store assembles stacks there); rows are read in place here."""
+
+  def check_flags(self, flags):
+    """Raises if the storage could not keep an added transition (the frame store's pool overflow)."""
+
+  def reset(self):
+    """Forgets the insert history before set_state() rewrites the rows."""
+
+  @property
+  def device_bytes(self):
+    """Bytes of device memory this store holds."""
+    return sum(t.numel() * t.element_size() for t in vars(self).values() if isinstance(t, torch.Tensor))
+
   def gather(self, d_slots, size):
     """`np.stack` of `get(ids)` (`replay.py:718-722`) on the device; returns device tensors."""
     dev = self.action.device
@@ -736,6 +758,95 @@ class _TransitionStore:
     s_tm1, a, r, d, s_t = [t.cpu().numpy() for t in tensors]
     shape = (len(a),) + self.obs_shape
     return type(structure)(s_tm1.view(self.obs_dtype).reshape(shape), a, r, d, s_t.view(self.obs_dtype).reshape(shape))
+
+
+class _FrameStore(_TransitionStore):
+  """Frame-deduplicated storage (DESIGN.md §3): observations are uint8 (H, W, S) stacks, every distinct (H, W) frame is
+  kept once in a ring of `frame_capacity` slots, and row = id % capacity holds the 2S frame slots of s_tm1 | s_t.  The
+  insert rule (include/dqn_zoo_b200.h, dz_frame_store) runs on the device in dz_replay_add; `gather` assembles the stacks
+  on the device, so everything returned is byte-identical to `_TransitionStore` after the same adds."""
+
+  def __init__(self, capacity, frame_capacity):
+    if int(frame_capacity) < 1:
+      raise ValueError('frame_capacity must be a positive integer, got %r' % (frame_capacity,))
+    super().__init__(capacity)
+    self.frame_capacity = int(frame_capacity)
+    self.batch_capacity = 0
+    self.batch_stage = None
+    self.state = None
+
+  def allocate(self, obs_shape, obs_dtype=np.uint8):
+    if self.obs_shape is not None:
+      return
+    shape, dtype = tuple(obs_shape), np.dtype(obs_dtype)
+    if len(shape) != 3 or dtype != np.uint8 or min(shape) < 1 or shape[2] > _lib.DZ_FRAME_MAX_STACK:
+      raise ValueError('frame store needs uint8 observations of shape (H, W, S) with S <= %d: %s %s'
+                       % (_lib.DZ_FRAME_MAX_STACK, shape, dtype))
+    if 2 * shape[2] * ((shape[0] * shape[1] + 15) // 16 * 16) > _lib.DZ_FRAME_MAX_STAGE_BYTES:
+      raise ValueError('frame store needs 2 * S * (H * W rounded up to 16) <= %d bytes: %s %s'
+                       % (_lib.DZ_FRAME_MAX_STAGE_BYTES, shape, dtype))
+    self.obs_shape, self.obs_dtype = shape, dtype
+    self.obs_bytes = int(np.prod(shape))
+    self.obs_stride = (self.obs_bytes + 15) // 16 * 16
+    h, w, self.stack = shape
+    self.frame_bytes = h * w
+    self.frame_stride = (self.frame_bytes + 15) // 16 * 16
+    dev, F, P = self.action.device, self.frame_capacity, 2 * self.stack
+    self.frames = torch.empty((F + 1, self.frame_stride), dtype=torch.uint8, device=dev)
+    self.frames[0].zero_()                              # slot 0: the zero frame of the padded stacks
+    self.row_frames = torch.zeros((max(self.capacity, 1), P), dtype=torch.int32, device=dev)
+    self.frame_hash = torch.zeros(F + 1, dtype=torch.int64, device=dev)   # uint64 bit patterns
+    self.frame_born = torch.full((F + 1,), -1, dtype=torch.int64, device=dev)
+    self.frame_last_ref = torch.full((F + 1,), -1, dtype=torch.int64, device=dev)
+    self.state = torch.empty(2 + _lib.DZ_FRAME_WINDOW * (1 + P), dtype=torch.int64, device=dev)
+    self.add_stage = torch.zeros((2, self.obs_stride), dtype=torch.uint8, device=dev)
+    self.reset()
+    self._allocate_batch_stage()
+
+  def _allocate_batch_stage(self):
+    if self.obs_shape is not None and self.batch_capacity:
+      self.batch_stage = torch.zeros((2, self.batch_capacity, self.obs_stride), dtype=torch.uint8,
+                                     device=self.action.device)
+
+  def reserve_batch(self, batch_size):
+    """The fused learner assembles each sampled batch into [2][batch_capacity][obs_stride] staging rows; the address
+    stays fixed once reserved, so captured CUDA graphs remain valid."""
+    if batch_size > self.batch_capacity:
+      self.batch_capacity = int(batch_size)
+      self._allocate_batch_stage()
+
+  def reset(self):
+    if self.state is not None:
+      self.state.fill_(-1)
+      self.state[:2] = 0
+
+  def check_flags(self, flags):
+    f = int(flags.item())
+    if f & _lib.DZ_FLAG_FRAME_POOL_FULL:
+      flags.fill_(f & ~_lib.DZ_FLAG_FRAME_POOL_FULL)
+      raise RuntimeError(_POOL_FULL_MESSAGE)
+
+  def fill_view(self, v):
+    super().fill_view(v)
+    if self.obs_shape is None:
+      return v
+    fs = v.frames
+    fs.d_frames, fs.d_row_frames = _ptr(self.frames), _ptr(self.row_frames)
+    fs.d_frame_hash, fs.d_frame_born, fs.d_frame_last_ref = (_ptr(self.frame_hash), _ptr(self.frame_born),
+                                                              _ptr(self.frame_last_ref))
+    fs.d_state, fs.d_add_stage, fs.d_batch_stage = _ptr(self.state), _ptr(self.add_stage), _ptr(self.batch_stage)
+    fs.num_frames, fs.frame_bytes, fs.frame_stride = self.frame_capacity, self.frame_bytes, self.frame_stride
+    fs.stack, fs.batch_capacity = self.stack, self.batch_capacity
+    return v
+
+  def fill_synthetic(self, n, seed, num_actions, discount, episode_length):
+    v = self.fill_view(_lib.ReplayView())
+    _lib.call('dz_replay_fill_synthetic_frames', C.byref(v), n, int(episode_length), int(seed), int(num_actions),
+              float(discount), _stream())
+
+
+def _make_store(capacity, frame_capacity):
+  return _TransitionStore(capacity) if frame_capacity is None else _FrameStore(capacity, frame_capacity)
 
 
 def _host_obs(x, store):
@@ -776,14 +887,17 @@ def _check_codec(encoder, decoder):
 class TransitionReplay:
   """Uniform replay with oldest-out eviction (`replay.py:120-200`), storage in HBM."""
 
-  def __init__(self, capacity: int, structure, random_state: np.random.RandomState, encoder=None, decoder=None):
+  def __init__(self, capacity: int, structure, random_state: np.random.RandomState, encoder=None, decoder=None, *,
+               frame_capacity: Optional[int] = None):
+    """`frame_capacity=F` stores every distinct frame of the (H, W, S) uint8 observation stacks once, in F slots
+    (`_FrameStore`); None keeps two full stacks per transition."""
     self._codec = _check_codec(encoder, decoder)
     self._capacity = capacity
     self._structure = structure
     self._random_state = random_state
     self._distribution = UniformDistribution(random_state=random_state)
     self._distribution._mirror.ensure(capacity)   # fixed address: captured CUDA graphs keep pointing at it
-    self._store = _TransitionStore(capacity)
+    self._store = _make_store(capacity, frame_capacity)
     self._live_ids = collections.deque()   # ids currently stored, oldest first (keys of the OrderedDict)
     self._t = 0
 
@@ -806,7 +920,8 @@ class TransitionReplay:
     v = self.device_view()
     first = patches[:4]
     _apply_index_record(v, first, slot=item_id % self._capacity, action=int(item[1]), reward=float(item[2]),
-                        discount=float(item[3]), h_s_tm1=s_tm1, h_s_t=s_t)
+                        discount=float(item[3]), h_s_tm1=s_tm1, h_s_t=s_t, item_id=item_id,
+                        oldest_live=self._live_ids[0] if self._live_ids else item_id)
     assert len(patches) <= 4
     self._live_ids.append(item_id)
     self._t += 1
@@ -817,6 +932,7 @@ class TransitionReplay:
     for i in ids:
       if not self._live_ids or not (self._live_ids[0] <= i <= self._live_ids[-1]):
         raise KeyError(i)
+    self._store.check_flags(self._store.flags)
     return self._store.get_rows(self._structure, np.asarray(ids, dtype=np.int64) % self._capacity)
 
   def sample_device(self, size: int):
@@ -834,6 +950,7 @@ class TransitionReplay:
   def sample(self, size: int):
     """`replay.py:158-165`."""
     _, _, tensors = self.sample_device(size)
+    self._store.check_flags(self._store.flags)
     return self._store.to_host_transition(self._structure, tensors)
 
   def ids(self) -> Iterable[int]:
@@ -847,11 +964,18 @@ class TransitionReplay:
   def capacity(self) -> int:
     return self._capacity
 
+  def reserve_batch(self, batch_size: int) -> None:
+    """Reserves the storage's staging for fused learner batches of up to `batch_size` (the agent calls it)."""
+    self._store.reserve_batch(batch_size)
+
   def get_state(self) -> Mapping[str, Any]:
     """`replay.py:179-187`: same keys; `storage` is a list of (id, Transition) with host arrays."""
     ids = list(self._live_ids)
     return {'storage': list(zip(ids, self.get(ids))) if ids else [], 't': self._t,
             'distribution': self._distribution.get_state()}
+
+  def _flags(self):
+    return self._store.flags
 
   def set_state(self, state: Mapping[str, Any]) -> None:
     """`replay.py:189-193`."""
@@ -861,6 +985,7 @@ class TransitionReplay:
 
   def check_valid(self) -> Tuple[bool, str]:
     """`replay.py:195-200`."""
+    self._store.check_flags(self._flags())
     if self._t < self.size:
       return False, 't should be >= storage size.'
     if set(self._live_ids) != set(self._distribution.ids()):
@@ -871,14 +996,15 @@ class TransitionReplay:
 def _restore_rows(rep, storage):
   """Rewrites device rows from a `storage` list of (id, item) (set_state)."""
   rep._live_ids = collections.deque(int(i) for i, _ in storage)
+  rep._store.reset()
   v = None
   for i, item in storage:
     s_tm1 = _host_obs(item[0], rep._store)
     s_t = _host_obs(item[4], rep._store)
     if v is None:
-      v = rep._store.fill_view(_lib.ReplayView())
+      v = rep.device_view()
     _apply_index_record(v, [], slot=int(i) % rep._capacity, action=int(item[1]), reward=float(item[2]),
-                        discount=float(item[3]), h_s_tm1=s_tm1, h_s_t=s_t)
+                        discount=float(item[3]), h_s_tm1=s_tm1, h_s_t=s_t, item_id=int(i), oldest_live=rep._live_ids[0])
 
 
 # ------------------------------------------------------------------------------------------------
@@ -891,7 +1017,9 @@ class PrioritizedTransitionReplay:
 
   def __init__(self, capacity: int, structure, priority_exponent: float,
                importance_sampling_exponent: Callable[[int], float], uniform_sample_probability: float,
-               normalize_weights: bool, random_state: np.random.RandomState, encoder=None, decoder=None):
+               normalize_weights: bool, random_state: np.random.RandomState, encoder=None, decoder=None, *,
+               frame_capacity: Optional[int] = None):
+    """`frame_capacity`: as for `TransitionReplay`."""
     self._codec = _check_codec(encoder, decoder)
     self._capacity = capacity
     self._structure = structure
@@ -901,7 +1029,7 @@ class PrioritizedTransitionReplay:
         uniform_sample_probability=uniform_sample_probability, random_state=random_state)
     self._importance_sampling_exponent = importance_sampling_exponent
     self._normalize_weights = normalize_weights
-    self._store = _TransitionStore(capacity)
+    self._store = _make_store(capacity, frame_capacity)
     self._live_ids = collections.deque()
     self._t = 0
 
@@ -941,7 +1069,8 @@ class PrioritizedTransitionReplay:
     _apply_index_record(v, patches[:4], tree_index=idx, leaf_value=float(leaf[0]), evict_index=evicted,
                         size_after=dist._sum_tree.size, slot=item_id % self._capacity, action=int(item[1]),
                         reward=float(item[2]), discount=float(item[3]), h_s_tm1=s_tm1, h_s_t=s_t,
-                        d_priority=d_priority, alpha=float(alpha))
+                        d_priority=d_priority, alpha=float(alpha), item_id=item_id,
+                        oldest_live=self._live_ids[0] if self._live_ids else item_id)
     assert len(patches) <= 4
     self._live_ids.append(item_id)
     self._t += 1
@@ -951,6 +1080,7 @@ class PrioritizedTransitionReplay:
     for i in ids:
       if i not in self._distribution._id_to_index:
         raise KeyError(i)
+    self._store.check_flags(self._flags())
     return self._store.get_rows(self._structure, np.asarray(ids, dtype=np.int64) % self._capacity)
 
   def sample_device(self, size: int):
@@ -967,6 +1097,7 @@ class PrioritizedTransitionReplay:
     ids, _, _, _, weights, tensors = self.sample_device(size)
     tr = self._store.to_host_transition(self._structure, tensors)
     w = weights.cpu().numpy()
+    self._store.check_flags(self._flags())
     self._distribution._sum_tree._raise_flags()
     if not np.isfinite(w).all():
       raise ValueError('Weights are not finite: %s.' % w)
@@ -983,6 +1114,13 @@ class PrioritizedTransitionReplay:
   @property
   def capacity(self) -> int:
     return self._capacity
+
+  def reserve_batch(self, batch_size: int) -> None:
+    """Reserves the storage's staging for fused learner batches of up to `batch_size` (the agent calls it)."""
+    self._store.reserve_batch(batch_size)
+
+  def _flags(self):
+    return self._distribution._sum_tree._flags
 
   @property
   def importance_sampling_exponent(self):
@@ -1003,6 +1141,7 @@ class PrioritizedTransitionReplay:
 
   def check_valid(self) -> Tuple[bool, str]:
     """`replay.py:762-768`."""
+    self._store.check_flags(self._flags())
     if self._t < self.size:
       return False, 't should be >= storage size.'
     if set(self._live_ids) != set(self._distribution.ids()):
@@ -1010,18 +1149,25 @@ class PrioritizedTransitionReplay:
     return self._distribution.check_valid()
 
 
-def bulk_fill_synthetic(rep, obs_shape, seed, num_actions, discount=0.99, priority=1.0):
+def bulk_fill_synthetic(rep, obs_shape, seed, num_actions, discount=0.99, priority=1.0, episode_length=1000):
   """Benchmark/test helper: brings `rep` (uniform or prioritized, empty) to the exact state it
   has after `capacity` sequential `add()`s of synthetic transitions (ids 0..C-1, priority
   `priority` each) without C host->device copies: contents are generated on the device
   (dz_replay_fill_synthetic, byte-identical to oracle/replay_oracle.py:synthetic_rows) and the
   host bookkeeping is written in closed form (allocation order of replay.py:457,499: id i gets
-  tree index C-1-i)."""
+  tree index C-1-i).
+
+  A frame store gets synthetic EPISODES instead (dz_replay_fill_synthetic_frames): `episode_length` 1-step transitions
+  each, a new iid frame per timestep, stacks zero-padded at episode start as processors.atari() pads them; the device
+  state equals that of the same sequential adds (oracle/frame_store_oracle.py:synthetic_fill)."""
   assert rep._t == 0 and rep.size == 0
   cap = rep._capacity
   rep._store.allocate(obs_shape, np.uint8)
-  v = rep._store.fill_view(_lib.ReplayView())
-  _lib.call('dz_replay_fill_synthetic', C.byref(v), 0, cap, int(seed), int(num_actions), float(discount), _stream())
+  if isinstance(rep._store, _FrameStore):
+    rep._store.fill_synthetic(cap, seed, num_actions, discount, episode_length)
+  else:
+    v = rep._store.fill_view(_lib.ReplayView())
+    _lib.call('dz_replay_fill_synthetic', C.byref(v), 0, cap, int(seed), int(num_actions), float(discount), _stream())
   rep._live_ids = collections.deque(range(cap))
   rep._t = cap
   dist = rep._distribution

@@ -79,11 +79,45 @@ int dz_sumtree_get(const double* d_nodes, int64_t first_leaf, int64_t size, cons
 #define DZ_FLAG_BAD_TARGET 4
 #define DZ_FLAG_ROOT_ZERO 8   /* fused PER step met root == 0 (reference would skip an RNG draw) */
 #define DZ_FLAG_NONFINITE_WEIGHT 16
+#define DZ_FLAG_FRAME_POOL_FULL 32   /* frame store: the ring slot an insert needed is still referenced by a live row */
 
 /* ------------------------------------------------------------------------------------------
  * R5/R6  Replay storage in HBM (replaces the OrderedDict storage of replay.py:120-200 and
  * :654-768; transition-major layout, see DESIGN.md §3)
  * ---------------------------------------------------------------------------------------- */
+
+/* Frame-deduplicated observation storage (DESIGN.md §3).  Observations are uint8 [H][W][S] stacks; each
+ * distinct [H][W] plane is kept once in a ring of F frame slots and a row holds 2S slot numbers instead of
+ * two stacks.  d_frames == NULL means the raw layout of dz_replay_view.d_obs.
+ *
+ * Insert rule (dz_replay_add): the 2S planes of s_tm1 | s_t are visited in that order; a plane reuses the
+ * most recently appended candidate whose hash AND bytes are equal, among the zero frame (slot 0), the
+ * frames appended by the last DZ_FRAME_WINDOW adds and the frames appended earlier in the same add;
+ * otherwise it is appended at slot 1 + appends % F.  A frame appended by add j is therefore referenced only
+ * by ids in [j, j + DZ_FRAME_WINDOW], and the ring slot at the head may be overwritten iff its last_ref is
+ * below the oldest live id.  When it may not, DZ_FLAG_FRAME_POOL_FULL is raised and the row's slots are
+ * set to -1 (its observations then read as zeros). */
+#define DZ_FRAME_WINDOW 16
+#define DZ_FRAME_MAX_STACK 8
+#define DZ_FRAME_MAX_STAGE_BYTES (200 * 1024)   /* 2 * stack * frame_stride: the insert de-interleaves both stacks
+                                                   into shared memory (84x84x4: 56,448 B) */
+typedef struct dz_frame_store {
+  uint8_t* d_frames;          /* [F + 1][frame_stride]; slot 0 is the all-zero frame                       */
+  int32_t* d_row_frames;      /* [capacity][2S]: frame slot of each plane of s_tm1 | s_t (-1: invalid row) */
+  uint64_t* d_frame_hash;     /* [F + 1] frame hash of each slot (slot 0: unused)                          */
+  int64_t* d_frame_born;      /* [F + 1] id of the add that appended the frame                             */
+  int64_t* d_frame_last_ref;  /* [F + 1] newest id whose row references the frame                          */
+  int64_t* d_state;           /* [2 + DZ_FRAME_WINDOW * (1 + 2S)]: appends so far, reserved, then one
+                                 window entry per add (id % DZ_FRAME_WINDOW): add id (-1: none) and the 2S
+                                 slots it appended in append order (-1 padded)                           */
+  uint8_t* d_add_stage;       /* [2][obs_stride]: the two stacks of the add in flight                      */
+  uint8_t* d_batch_stage;     /* [2][batch_capacity][obs_stride]: stacks assembled for the fused learner   */
+  int64_t num_frames;         /* F */
+  int64_t frame_bytes;        /* H * W */
+  int64_t frame_stride;       /* frame_bytes rounded up to 16 */
+  int32_t stack;              /* S <= DZ_FRAME_MAX_STACK */
+  int32_t batch_capacity;
+} dz_frame_store;
 
 typedef struct dz_replay_view {
   uint8_t* d_obs;        /* [capacity][2][obs_stride]: s_tm1 then s_t of each transition      */
@@ -102,6 +136,7 @@ typedef struct dz_replay_view {
   /* uniform replay only */
   int64_t* d_ids;        /* `UniformDistribution._ids` (replay.py:49): dense list of ids      */
   int32_t* d_flags;      /* sticky error flags (1 int32)                                      */
+  dz_frame_store frames; /* frame-deduplicated storage; frames.d_frames == NULL: d_obs holds raw rows */
 } dz_replay_view;
 
 /* One `add` (replay.py:142-151 / :690-699) after the HOST has done the O(1) integer
@@ -126,6 +161,8 @@ typedef struct dz_add_record {
                                 max_seen_priority, rainbow/agent.py:148-149) instead of leaf_value;
                                 leaf = ((double)*d_priority) ** alpha in float64, exact for alpha 0.5 / 1 */
   double alpha;
+  int64_t item_id;           /* frame store only: id of the transition being added            */
+  int64_t oldest_live;       /* frame store only: oldest live id after this add's eviction    */
 } dz_add_record;
 
 /* s_tm1 / s_t sources may be HOST arrays or DEVICE buffers (cudaMemcpyDefault; NULL = leave the row's bytes). */
@@ -138,6 +175,19 @@ int dz_replay_add(const dz_replay_view* view, const dz_add_record* rec, const ui
  * `discount` w.p. .99 else 0 (SURVEY §8(d)). */
 int dz_replay_fill_synthetic(const dz_replay_view* view, int64_t row0, int64_t n, uint64_t seed,
                              int32_t num_actions, double discount, void* stream);
+
+/* Frame-store counterpart of dz_replay_fill_synthetic: brings an EMPTY frame store to the exact state that n
+ * sequential adds (ids 0..n-1, rows 0..n-1) of 1-step transitions of synthetic episodes produce.  Episodes are
+ * `episode_length` transitions long; every timestep shows a new iid frame (splitmix64 of seed and its append
+ * index, byte-identical to oracle/frame_store_oracle.py:synthetic_frame); stacks are padded with trailing zero
+ * planes at episode start (processors.py:497-504).  Scalars are those of dz_replay_fill_synthetic.  Needs
+ * frame_bytes % 8 == 0 and F >= the frames appended (n + ceil(n / episode_length)). */
+int dz_replay_fill_synthetic_frames(const dz_replay_view* view, int64_t n, int64_t episode_length, uint64_t seed,
+                                    int32_t num_actions, double discount, void* stream);
+/* The insert rule's 64-bit frame hash of n host bytes, evaluated on the HOST by the same source the kernels
+ * compile; tests only.  hash = mix64(n ^ K0) + sum_k mix64(w_k ^ k * K1) mod 2^64 over the little-endian 8-byte
+ * words w_k of the zero-padded bytes (mix64 = the splitmix64 finalizer; constants in csrc/dz_frames.cu). */
+int dz_test_frame_hash(const uint8_t* h_bytes, int64_t n, uint64_t* out);
 
 /* Per-step sampling inputs that live in device memory so that a captured CUDA graph can be
  * replayed: the three host RandomState draws of replay.py:551-567 plus the scalars that
@@ -259,7 +309,8 @@ int dz_learner_update(dz_learner* l, const dz_batch* batch, const dz_update_outp
                       void* stream);
 
 /* The whole `_learn()` (rainbow/agent.py:181-198) in one enqueue: sample -> (rows addressed in
- * place) -> update -> priority write-back.  `d_max_seen_priority` ([1] float32, device) is
+ * place; with a frame store, stacks assembled into replay->frames.d_batch_stage, DZ_EINVAL when the
+ * batch exceeds its batch_capacity) -> update -> priority write-back.  `d_max_seen_priority` ([1] float32, device) is
  * updated as max(old, batch max) (rainbow/agent.py:196-197). */
 typedef struct dz_learn_io {
   dz_sample_inputs sample_in;
